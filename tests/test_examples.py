@@ -36,6 +36,9 @@ def test_allen_cahn_piratenet_example_trains_two_iterations(monkeypatch, arch):
 
     lib = B.Library(build())
     monkeypatch.setattr(B, "_default", lib)
+    # the emulated library reads host memory: the Solver must keep the model and data on the host even where a GPU is
+    # visible (it moves them to CUDA whenever one is)
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)
 
     def cpu_step(self):  # FlatAdam.step without the device guard, on the emulated library
         p = self.model.flat
