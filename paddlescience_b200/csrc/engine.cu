@@ -359,15 +359,18 @@ extern "C" int ppsci_b200_plan_create(const ppsci_plan_spec* s, ppsci_plan** out
   }
   P->use_tc = tc_plan_supported(P->spec, P->C, P->kmax) && s->backend != 1 && !s->gated &&
               s->act != PPSCI_ACT_STAN && s->act != PPSCI_ACT_SWISH_B;
+  // the tensor-core kernels apply s.act to every hidden layer, layer 1 included (fill_act, the fused forward / dx
+  // chains): a different first-layer activation (a Fourier embedding's sin) runs on the CUDA-core kernels
+  if (s->act_first >= 0 && s->act_first != s->act) P->use_tc = false;
 #ifdef PPSCI_EMUL
-  if (s->act_first >= 0 && s->act_first != s->act) P->use_tc = false;  // one activation across the fused layers
   if (s->backend != 2) P->use_tc = false;  // the emulated tensor-core kernels (1,024 OS threads per CTA pair) run on request only
 #endif
   if (const char* m = getenv("PPSCI_B200_TC_MASK")) P->tc_mask = atoi(m);
   if (s->backend == 2 && !P->use_tc) {
     delete P;
-    return fail("plan_create: backend=2 (tcgen05) requested but the plan is not eligible "
-                "(needs f32, tanh, hidden widths in {128,256}, order<=2)");
+    return fail("plan_create: backend=2 (tcgen05) requested but the plan is not eligible (needs f32, no gated layers, "
+                "one activation across all hidden layers and not stan / swish, and at least one layer after the first "
+                "with K a multiple of 32 up to 1024 and N a multiple of 32 up to 256)");
   }
 
   auto up = [&](const void* src, size_t bytes, void** dst) -> cudaError_t {

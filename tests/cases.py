@@ -64,7 +64,8 @@ def _first_order_exprs():
 
 
 CASES = {
-    # name: dict(in_keys, out_keys, hidden, act, exprs, dtype, periods, reduction, weights, labels_rand, oracle_exprs, ranges, chunk)
+    # name: dict(in_keys, out_keys, hidden, act, exprs, dtype, periods, reduction, weights, labels_rand, oracle_exprs, ranges, chunk,
+    #            param_scale)
     "ns_f32": dict(in_keys=("x", "y"), out_keys=("u", "v", "p"), hidden=[20, 20], act="tanh",
                    exprs=lambda: O.navier_stokes_expr(0.01, 1.0, 2, False), dtype=torch.float32),
     "laplace_f32_sum_w": dict(in_keys=("x", "y"), out_keys=("u",), hidden=[20] * 4, act="tanh",
@@ -239,6 +240,8 @@ def run_case(name, n: int, library=None, device="cpu", backend: int = 0, seed: i
         params = torch.cat([params, O.xavier_uniform_params([om.widths[0], om.widths[1]], 2, torch.float64),
                             O.xavier_uniform_params([om.widths[0], om.widths[1]], 3, torch.float64)])
     params = (params + 0.1 * torch.randn_like(params))
+    if c.get("param_scale"):  # weights and biases away from the init scale (a trained or a shrunk network)
+        params = params * float(c["param_scale"])
     if c.get("trainable_act"):  # Stan.beta per unit / Swish.beta per layer, behind the layers (1 at start in the reference)
         params = torch.cat([params, 1.0 + 0.2 * torch.randn(sum(om.beta_len), dtype=torch.float64)])
     if c.get("siren_init"):  # weights on the scale Siren's initialisers use (sqrt(6 / in) / w0, activation.py:103-136)
